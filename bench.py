@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's own CPU implementation of the same workload
+    python bench.py ... --dump-outputs DIR    # also write what the last timed step computed, as DIR/<name>.npy
 
 --config (default hg_fpd = BASELINE.json configs[1] at N=1, configs[2] at N>1):
     hg_fpd     student hourglass s4 f128 + frozen teacher s8 f256, FPD loss, 256x256, batch 32/GPU        (configs[1], [2])
@@ -266,7 +267,12 @@ class CpuReference:
         else:
             self.student.eval()
             self.boxes = synthetic_boxes(1024, 1)
-            self.dec = R.decode() if self.kind == "reference" else None
+            if self.kind == "reference":
+                inf, tr, ns = R.decode()
+                self.dec = (inf.get_max_preds, tr.flip_back, ns["nms"])
+            else:
+                from oracle import decode_oracle as D
+                self.dec = (D.get_max_preds, D.flip_back, D.nms)
 
     def _port_init(self, c):
         """oracle port (hourglass only): functional restatement driven from a state_dict."""
@@ -326,22 +332,28 @@ class CpuReference:
         self.opt.step()
         return loss.item()
 
+    def _forward(self, x):
+        if self.kind == "port":
+            from oracle import hourglass_oracle as O
+            return O.hourglass_net(self.s_sd, x, self.c["student"][1], training=False)
+        return self.student(x)
+
     def _infer(self):
         """function.py:212-240 + inference.get_max_preds + numpy nms, on the CPU."""
         import numpy as np
         import torch
-        inf, tr, ns = self.dec
+        get_max_preds, flip_back, nms = self.dec
         with torch.no_grad():
-            out = self.student(self.x)
+            out = self._forward(self.x)
             out = out[-1] if isinstance(out, list) else out
             xf = torch.from_numpy(np.flip(self.x.numpy(), 3).copy())
-            of = self.student(xf)
+            of = self._forward(xf)
             of = of[-1] if isinstance(of, list) else of
-            of = torch.from_numpy(tr.flip_back(of.numpy(), MPII_FLIP_PAIRS).copy())
+            of = torch.from_numpy(flip_back(of.numpy(), MPII_FLIP_PAIRS).copy())
             of[:, :, :, 1:] = of.clone()[:, :, :, 0:-1]
             out = (out + of) * 0.5
-        preds, maxvals = inf.get_max_preds(out.numpy())
-        keep = ns["nms"](self.boxes, 0.6)
+        preds, maxvals = get_max_preds(out.numpy())
+        keep = nms(self.boxes, 0.6)
         return float(maxvals.sum()) + len(keep)
 
 
@@ -435,6 +447,25 @@ def time_dominant_kernel(B, roof):
     return ms, flops
 
 
+DUMP_MAX_ELEMS = 4 << 20     # per array: at most 16 MB, so that one dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy: float32 as it is, anything else (integer indices) as float64, which holds
+    it exactly. An array of more than DUMP_MAX_ELEMS entries is flattened and reduced to a fixed sample of that many: the
+    same seeded, sorted index set on every run, so that dumps of two builds compare entry for entry."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu()
+        if a.numel() > DUMP_MAX_ELEMS:
+            pick = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            a = a.reshape(-1)[pick]
+        a = a.numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def build_models(name, dev):
     import torch
     import fpd_b200  # noqa: F401
@@ -500,12 +531,19 @@ def run_b200(args, rank, local_rank, world):
         d2h = 12
         launches = lambda: int(step.launches_per_step or 0)                  # noqa: E731
         final = lambda: float(loss_host[2])                                   # noqa: E731
+        # the step's result: its losses (pose, kd, total), the gradient it applied and the student's weights and BatchNorm
+        # running statistics after its update (flat, in module order)
+        outputs = lambda: {"losses": step.losses, "grad": step.flat.grad, "weights": step.flat.flat,   # noqa: E731
+                           "bn_running": torch.cat([b.reshape(-1) for b in student.buffers() if b.is_floating_point()])}
     else:
         from fpd_b200.infer_step import FlipTestInference
         boxes = torch.from_numpy(synthetic_boxes(1024, 1)).to(dev)
         inf = FlipTestInference(student, MPII_FLIP_PAIRS, shift_heatmap=True, flip_test=c.get("flip", True),
                                 use_graph=graph_ok, want_avg=False)
-        run_dev = lambda: inf(xd, boxes, 0.6)                                # noqa: E731
+        last = {}
+
+        def run_dev():
+            last["r"] = inf(xd, boxes, 0.6)
         idx_host = torch.empty(B, c["J"], dtype=torch.int32).pin_memory()
         max_host = torch.empty(B, c["J"], dtype=torch.float32).pin_memory()
         keep_host = torch.empty(1024, dtype=torch.int32).pin_memory()
@@ -519,6 +557,8 @@ def run_b200(args, rank, local_rank, world):
         d2h = idx_host.numel() * 4 + max_host.numel() * 4 + keep_host.numel() * 4
         launches = lambda: int(getattr(inf, "launches", 0))                  # noqa: E731
         final = lambda: float(max_host.sum())                                # noqa: E731
+        outputs = lambda: {"idx": last["r"]["idx"], "maxval": last["r"]["maxval"],                   # noqa: E731
+                           "nms_keep": last["r"]["nms_keep"][:int(last["r"]["nms_num"])]}
 
     def barrier():
         if world > 1:
@@ -546,6 +586,8 @@ def run_b200(args, rank, local_rank, world):
         sampler.start()
     ms_total = timed(run_dev, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs())
     ms_step = ms_total / args.steps
     value = world * B / (ms_step / 1000.0)
 
@@ -640,6 +682,8 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="images per GPU (default: the config's)")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

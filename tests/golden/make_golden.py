@@ -1,7 +1,7 @@
 """Generate the golden vectors under tests/golden/ by running the REAL reference
 (/root/reference, read-only) on seeded synthetic inputs. Run in the build container only:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [decode2 | resnet | hg_modes | resnet_layout]
 
 The reference has no tests / fixtures of its own (SURVEY.md section 4), so these vectors -- outputs of its
 own lib/models/hourglass.py, lib/core/loss.py, lib/core/inference.py, lib/utils/transforms.py and
@@ -218,11 +218,58 @@ def main_resnet():
     print("resnet_small.npz", os.path.getsize(os.path.join(OUT, "resnet_small.npz")))
 
 
+def main_hg_modes():
+    """Section 8: the reference's lib/models/hourglass.py, s=1 f=64 with its default initialisation under
+    torch.manual_seed(3), then x = torch.randn(2, 3, 64, 64): the first output in train mode, and in eval mode with the
+    running statistics that train-mode pass left (stored too, concatenated in state_dict order). The weights and x are
+    regenerated from the seed by the test -- the network is too large to commit -- and pinned by their float64 sums."""
+    torch.set_num_threads(4)
+    hg = load("ref_hourglass", "lib/models/hourglass.py")
+    torch.manual_seed(3)
+    net = hg.get_pose_net(cfg(64, 1), True)
+    x = torch.randn(2, 3, 64, 64)
+    sd = net.state_dict()
+    save = {"x_sum": np.float64(x.double().sum().item()), "keys": np.array(list(sd.keys())),
+            "sums": np.array([v.double().sum().item() for v in sd.values()], np.float64)}
+    with torch.no_grad():
+        net.train()
+        save["out_train"] = net(x)[0].numpy()
+        save["running_after_train"] = torch.cat([v.reshape(-1) for k, v in net.state_dict().items()
+                                                 if "running" in k]).numpy()
+        net.eval()
+        save["out_eval"] = net(x)[0].numpy()
+    np.savez_compressed(os.path.join(OUT, "hg_s1f64_modes.npz"), **save)
+    print("hg_s1f64_modes.npz", os.path.getsize(os.path.join(OUT, "hg_s1f64_modes.npz")))
+
+
+def main_resnet_layout():
+    """Section 9: the state_dict layout (keys in order, shapes) of the reference's pose_resnet for both RESNET_CASES and,
+    with the shipped 3 x 256-filter 4x4 deconv head, for the remaining depths of its resnet_spec; and the block counts of
+    resnet_spec itself."""
+    R = load("ref_pose_resnet", "lib/models/pose_resnet.py")
+    save = {}
+    for depth, (_, blocks) in R.resnet_spec.items():
+        save["resnet_spec/%d" % depth] = np.array(blocks, np.int64)
+    cases = dict(RESNET_CASES)
+    for depth in (34, 101, 152):
+        cases["d%d" % depth] = (depth, 16, (256, 256, 256), (4, 4, 4), 1, False)
+    for tag, case in cases.items():
+        sd = R.get_pose_net(resnet_cfg(*case), is_train=False).state_dict()
+        save[tag + "/keys"] = np.array(list(sd.keys()))
+        save[tag + "/shapes"] = np.array([",".join(str(n) for n in v.shape) for v in sd.values()])
+    np.savez_compressed(os.path.join(OUT, "resnet_layout.npz"), **save)
+    print("resnet_layout.npz", os.path.getsize(os.path.join(OUT, "resnet_layout.npz")))
+
+
 def main():
     if len(sys.argv) > 1 and sys.argv[1] == "decode2":
         return main_decode2()
     if len(sys.argv) > 1 and sys.argv[1] == "resnet":
         return main_resnet()
+    if len(sys.argv) > 1 and sys.argv[1] == "hg_modes":
+        return main_hg_modes()
+    if len(sys.argv) > 1 and sys.argv[1] == "resnet_layout":
+        return main_resnet_layout()
     torch.set_num_threads(4)
     hg = load("ref_hourglass", "lib/models/hourglass.py")
     loss_mod = load("ref_loss", "lib/core/loss.py")

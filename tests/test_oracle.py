@@ -1,6 +1,5 @@
 """CPU suite (no GPU): pins the oracle (oracle/) against golden vectors produced by the real reference
-(tests/golden/make_golden.py) and -- when /root/reference exists -- against the live reference modules."""
-import importlib.util
+(tests/golden/make_golden.py)."""
 import os
 import sys
 import types
@@ -13,7 +12,6 @@ from oracle import decode_oracle as D
 from oracle import hourglass_oracle as O
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REF = "/root/reference"
 
 
 def _load(name):
@@ -102,24 +100,36 @@ def test_decode_and_nms_match_reference_golden():
     assert D.nms(np.zeros((0, 5), np.float32), 0.5) == []
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="live reference only exists in the build container")
-def test_oracle_matches_live_reference_module():
+def test_oracle_matches_reference_module_golden():
+    """The reference's hourglass module at its default initialisation (tests/golden/hg_s1f64_modes.npz), train and eval
+    mode. The drop-in module draws the same weights from the same seed; their sums pin that."""
+    import fpd_b200  # noqa: F401
+    from fpd_b200.lib.models import hourglass as H
     torch.set_num_threads(4)
-    spec = importlib.util.spec_from_file_location("ref_hg_live", os.path.join(REF, "lib/models/hourglass.py"))
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
+    g = _load("hg_s1f64_modes.npz")
     NS = types.SimpleNamespace
     cfg = NS(MODEL=NS(EXTRA=NS(NUM_FEATURES=64, NUM_STACKS=1, NUM_BLOCKS=1), NUM_JOINTS=16))
     torch.manual_seed(3)
-    net = m.get_pose_net(cfg, True)
+    sd = H.get_pose_net(cfg, True).state_dict()
     x = torch.randn(2, 3, 64, 64)
-    for training in (True, False):
-        net.train(training)
-        sd = {k: v.clone() for k, v in net.state_dict().items()}
-        with torch.no_grad():
-            ref = net(x)
-            got = O.hourglass_net(sd, x, num_stacks=1, training=training)
-        assert _rel(got[0], ref[0]) < 1e-5
+    assert list(sd.keys()) == [str(k) for k in g["keys"]]
+    sums = np.array([v.double().sum().item() for v in sd.values()])
+    np.testing.assert_allclose(sums, g["sums"], rtol=1e-9, atol=1e-9)
+    assert abs(x.double().sum().item() - float(g["x_sum"])) < 1e-9 * x.numel()
+    with torch.no_grad():
+        got = O.hourglass_net({k: v.clone() for k, v in sd.items()}, x, num_stacks=1, training=True)
+        assert _rel(got[0], g["out_train"]) < 1e-5
+        # eval mode with the running statistics the reference's train-mode pass left
+        after = torch.from_numpy(g["running_after_train"])
+        sd_eval, off = {}, 0
+        for k, v in sd.items():
+            if "running" in k:
+                v = after[off:off + v.numel()].reshape(v.shape)
+                off += v.numel()
+            sd_eval[k] = v
+        assert off == after.numel()
+        got = O.hourglass_net(sd_eval, x, num_stacks=1, training=False)
+        assert _rel(got[0], g["out_eval"]) < 1e-5
 
 
 def test_dropin_module_state_dict_matches_reference_keys(train_gold):
@@ -253,30 +263,30 @@ def test_resnet_dropin_matches_reference_layout_and_refuses_cpu():
     assert type(net.deconv_layers[0]).__name__ == "ConvTranspose2d" and net.deconv_layers[0].bias is None
     with pytest.raises(RuntimeError, match="no CPU fallback|CUDA"):
         net(torch.zeros(1, 3, 64, 64))
-    if os.path.isdir(REF):        # live reference: every depth of resnet_spec has the same keys / shapes
-        spec = importlib.util.spec_from_file_location("ref_pose_resnet_t", os.path.join(REF, "lib/models/pose_resnet.py"))
-        R = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(R)
-        from fpd_b200.lib.models import pose_resnet as M
-        assert {k: v[1] for k, v in M.resnet_spec.items()} == {k: v[1] for k, v in R.resnet_spec.items()}
-        for tag in ("r18", "r50"):
-            a = R.get_pose_net(_resnet_cfg(tag), is_train=False).state_dict()
-            b = M.get_pose_net(_resnet_cfg(tag), is_train=False).state_dict()
-            assert list(a.keys()) == list(b.keys()) and all(a[k].shape == b[k].shape for k in a)
-        for depth in (34, 101, 152):          # the shipped d256x3 head on the remaining depths of resnet_spec
-            cfg = _resnet_cfg("r50")
-            cfg.MODEL.EXTRA.NUM_LAYERS = depth
-            cfg.MODEL.EXTRA.NUM_DECONV_FILTERS = [256, 256, 256]
-            a = R.get_pose_net(cfg, is_train=False).state_dict()
-            b = M.get_pose_net(cfg, is_train=False).state_dict()
-            assert list(a.keys()) == list(b.keys()) and all(a[k].shape == b[k].shape for k in a), depth
-        # init_weights without a checkpoint (pose_resnet.py:229-247): N(0, 0.001) convs / deconvs, unit BatchNorm
-        cfg = _resnet_cfg("r18")
-        cfg.MODEL.INIT_WEIGHTS = True
-        net = M.get_pose_net(cfg, is_train=True)
-        assert 5e-4 < net.layer2[0].conv1.weight.std().item() < 2e-3
-        assert 5e-4 < net.deconv_layers[0].weight.std().item() < 2e-3 and float(net.deconv_layers[0].bias.detach().abs().max()) == 0.0
-        assert torch.equal(net.deconv_layers[1].weight, torch.ones_like(net.deconv_layers[1].weight))
+    # every depth of the reference's resnet_spec has the same keys / shapes (tests/golden/resnet_layout.npz)
+    g = _load("resnet_layout.npz")
+    from fpd_b200.lib.models import pose_resnet as M
+    assert {k: list(v[1]) for k, v in M.resnet_spec.items()} == {
+        int(k.split("/")[1]): g[k].tolist() for k in g if k.startswith("resnet_spec/")}
+
+    def layout(tag, cfg):
+        sd = M.get_pose_net(cfg, is_train=False).state_dict()
+        assert list(sd.keys()) == [str(k) for k in g[tag + "/keys"]], tag
+        assert [",".join(str(n) for n in v.shape) for v in sd.values()] == [str(s) for s in g[tag + "/shapes"]], tag
+    for tag in ("r18", "r50"):
+        layout(tag, _resnet_cfg(tag))
+    for depth in (34, 101, 152):          # the shipped d256x3 head on the remaining depths of resnet_spec
+        cfg = _resnet_cfg("r50")
+        cfg.MODEL.EXTRA.NUM_LAYERS = depth
+        cfg.MODEL.EXTRA.NUM_DECONV_FILTERS = [256, 256, 256]
+        layout("d%d" % depth, cfg)
+    # init_weights without a checkpoint (pose_resnet.py:229-247): N(0, 0.001) convs / deconvs, unit BatchNorm
+    cfg = _resnet_cfg("r18")
+    cfg.MODEL.INIT_WEIGHTS = True
+    net = M.get_pose_net(cfg, is_train=True)
+    assert 5e-4 < net.layer2[0].conv1.weight.std().item() < 2e-3
+    assert 5e-4 < net.deconv_layers[0].weight.std().item() < 2e-3 and float(net.deconv_layers[0].bias.detach().abs().max()) == 0.0
+    assert torch.equal(net.deconv_layers[1].weight, torch.ones_like(net.deconv_layers[1].weight))
 
 
 @pytest.mark.parametrize("k,pad,outpad", [(4, 1, 0), (3, 1, 1), (2, 0, 0)])
